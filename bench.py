@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W                 # this repo's B200 engine, BASELINE configs[1]
     python bench.py --config c3|c4|c5 --gpus N ...                # the other BASELINE configs (528^2 / 8 characters / 1024^2 stage 1)
     python bench.py --impl reference --gpus N --steps K ...       # the reference's CPU path (oracle port) on the host cores
+    python bench.py --gpus 1 --steps K --dump-outputs DIR         # also save what the timed path returned in its last step
 
 One *step* = one pass of stage 1 -> uint8 -> edge burn-in -> stage 2 -> uint8 RGBA over the rank's synthetic
 frame stack.  With N > 1 (torchrun, one rank per GPU) every rank owns its own frame range, weights are broadcast
@@ -37,6 +38,7 @@ if ROOT not in sys.path:
 METRIC = "stylized frames/sec @512x512 (stage1+stage2)"
 UNIT = "frames/s"
 TOL = 1e-3          # BASELINE.json north_star: max-abs fp32 against the reference's own forward
+DUMP_BYTES = 60 * 10**6   # float32 payload of --dump-outputs: with the .npy headers the dump stays under 64 MB
 
 CONFIGS = {
     # name: (workload description, frame size, total frames (None = per-GPU), characters, stage-1 only, scaling)
@@ -341,7 +343,13 @@ def main():
     ap.add_argument("--no-gpu-baseline", action="store_true")
     ap.add_argument("--no-fast", action="store_true", help="skip the secondary single-pass fp16 measurement")
     ap.add_argument("--no-parity-gate", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the uint8 RGBA frames the timed path returned in its last step as "
+                         "DIR/rgba_char<c>.npy (float32 [k,H,W,4]; rank 0; k frames per character chosen by a fixed seed "
+                         "so that the dump stays under 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -414,21 +422,25 @@ def main():
         return {c: StylizationPipeline(weights[c][0], None if stage1_only else weights[c][1], dev, precision=precision,
                                        batch=args.batch) for c in my_chars}
 
+    last = {}                                             # character -> RGBA frames of the last timed device-resident step
+
     def measure(pipes, host: bool):
-        def fn():
+        def fn(keep=False):
             for c in my_chars:
                 st = stacks[c]
                 if host:
                     pipes[c].run_host(*st["host"], st["out"])
                 else:
-                    pipes[c].run(*st["dev"])
+                    out = pipes[c].run(*st["dev"])
+                    if keep:
+                        last[c] = out
         for _ in range(args.warmup):
             fn()
         barrier()
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
-        for _ in range(args.steps):
-            fn()
+        for i in range(args.steps):
+            fn(keep=i == args.steps - 1)
         ev1.record()
         barrier()
         ms = torch.tensor([ev0.elapsed_time(ev1)], device=dev)
@@ -497,6 +509,14 @@ def main():
         sampler.start()
     ms_total = measure(pipes, host=False)
     clocks = sampler.stop() if rank == 0 else None
+    if rank == 0 and args.dump_outputs:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        per_char = DUMP_BYTES // len(my_chars) // (S * S * 4 * 4)
+        for c in my_chars:
+            idx = np.sort(np.random.default_rng(c).choice(frames_of[c], min(frames_of[c], per_char), replace=False))
+            np.save(os.path.join(args.dump_outputs, "rgba_char%d.npy" % c),
+                    last[c][torch.from_numpy(idx).to(dev)].float().cpu().numpy())
+    last.clear()
     ms_e2e = measure(pipes, host=True)
     fps = all_frames * args.steps / (ms_total / 1e3)
     fps_e2e = all_frames * args.steps / (ms_e2e / 1e3)
@@ -530,6 +550,7 @@ def main():
             fast["note"] = ("single-pass fp16 operands / fp32 accumulate: same operand class as the reference's default GPU "
                             "path (cuDNN TF32, 10-bit mantissa; see gpu_baseline.library_default.max_abs_err_vs_fp32)")
         del pipes_f
+        last.clear()
         torch.cuda.empty_cache()
 
     gpu_base = None

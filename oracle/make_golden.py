@@ -16,7 +16,10 @@ What is recorded (all seeded, see drawingspinup_b200/synth.py):
   * ``DatasetFullImages.__getitem__`` (data.py:23-47) incl. the stage-2 edge burn-in, via real PNGs;
   * ``to_image_space`` (custom_transforms.py:7-8) known answers;
   * ``pos2edge`` (run_render.py:31-57; the function is extracted with ``ast`` because importing the
-    module needs Blender-side packages).
+    module needs Blender-side packages);
+  * the state-dict layout (keys in order, shapes, dtypes) of the models ``build_model`` (trainers.py:33-35)
+    makes for both stages, and the PNG frames the unmodified ``test_stage1.py`` / ``test_stage2.py`` write
+    for a synthetic 3-frame character (``GOLDEN_ONLY=scripts`` records just these two files).
 """
 from __future__ import annotations
 
@@ -52,7 +55,60 @@ def _no_cuda(fn, *a, **k):
         torch.Tensor.cuda = orig
 
 
+def reference_scripts():
+    """Layout of the models ``build_model`` returns, and one run of the unmodified stage-1 and stage-2 scripts on the
+    CPU (the YAML's ``device: cuda:0`` is replaced by ``cpu`` as the configs are read) over a synthetic character whose
+    checkpoints are ``synth.make_state_dict(stage, out_gain=0.25)``.  Stage 2 reads the PNGs stage 1 wrote."""
+    import json
+    import runpy
+    import yaml
+    from PIL import Image
+    import training.trainers as rt
+    layout = {}
+    for name in ("GeneratorJ_RIC", "GeneratorJ"):
+        sd = rt.build_model(name, dict(ARGS), "cpu").state_dict()
+        layout[name] = [[k, list(v.shape), str(v.dtype)] for k, v in sd.items()]
+    with open(os.path.join(OUT, "reference_state_dict_layout.json"), "w") as f:
+        json.dump({"args": ARGS, "models": layout}, f, indent=0)
+
+    uid, action, n, h, w, out_gain = "synthetic0001", "dab", 3, 64, 48, 0.25
+    sds = tuple(synth.to_torch_state_dict(synth.make_state_dict(s, out_gain=out_gain)) for s in (1, 2))
+    real_load, cwd, argv = yaml.load, os.getcwd(), list(sys.argv)
+
+    def cpu_config(stream, Loader):
+        cfg = real_load(stream, Loader=Loader)
+        cfg["job"]["device"] = "cpu"
+        return cfg
+
+    with tempfile.TemporaryDirectory() as tmp:
+        work = os.path.join(tmp, "3_style_translator")
+        os.makedirs(work)
+        for name in ("test_stage1.py", "test_stage2.py", "training", "configs"):
+            os.symlink(os.path.join(REF, name), os.path.join(work, name))
+        root = os.path.join(tmp, "dataset", "AnimatedDrawings", "preprocessed")     # config_stage1.yaml root_dir
+        color, pos, edge = synth.write_character_tree(root, uid, {action: n}, h, w, seed=5, state_dicts=sds)[action]
+        yaml.load = cpu_config
+        try:
+            os.chdir(work)
+            for script in ("test_stage1.py", "test_stage2.py"):
+                sys.argv = [script, "--uid", uid]
+                _no_cuda(runpy.run_path, os.path.join(work, script), run_name="__main__")
+        finally:
+            yaml.load, sys.argv = real_load, argv
+            os.chdir(cwd)
+        base = os.path.join(root, uid, "mesh", "blender_render", action)
+        res = {d: np.stack([np.array(Image.open(os.path.join(base, d, "%04d.png" % i))) for i in range(n)])
+               for d in ("res_stage1_mask_pos", "res_stage2_mask_pos_edge")}
+    np.savez_compressed(os.path.join(OUT, "reference_scripts.npz"), color=color, pos=pos, edge=edge,
+                        stage1=res["res_stage1_mask_pos"], stage2=res["res_stage2_mask_pos_edge"],
+                        out_gain=np.array(out_gain))
+    print("reference script frames", {k: v.shape for k, v in res.items()})
+
+
 def main():
+    if os.environ.get("GOLDEN_ONLY", "") == "scripts":
+        os.makedirs(OUT, exist_ok=True)
+        return reference_scripts()
     import training.models as rm
     from training.data import DatasetFullImages
     from training.custom_transforms import to_image_space
@@ -147,6 +203,7 @@ def main():
             cv2.imwrite(path, p64[i][..., [2, 1, 0, 3]])       # RGBA array -> BGRA file order
             edges.append(ns["pos2edge"](path))
     np.savez_compressed(os.path.join(OUT, "pos2edge.npz"), pos=p64, edges=np.stack(edges))
+    reference_scripts()
     print("golden fixtures written to", OUT)
 
 

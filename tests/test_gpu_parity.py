@@ -538,55 +538,28 @@ def test_multi_gpu_shard_equivalence(dev):
     assert torch.equal(torch.cat(outs), single)
 
 
-# ------------------------------------------------------------------ the UNMODIFIED reference scripts on the engine
-def _reference_dir():
-    for cand in (os.environ.get("DSU_REFERENCE_DIR"), "/root/reference/3_style_translator",
-                 os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "_refcopy", "3_style_translator")):
-        if cand and os.path.exists(os.path.join(cand, "test_stage1.py")):
-            return cand
-    return None
-
-
-def test_unmodified_reference_scripts_run_on_the_engine(dev, tmp_path):
-    """SURVEY.md section 4 item 4: `python -m drawingspinup_b200.run <reference>/test_stage1.py --uid u`, then test_stage2.py, on a
-    synthetic <uid> tree; the PNGs the reference's own loop writes are compared with the oracle chain (<= 1 LSB).
-    The scripts, training/*.py and configs/*.yaml are used IN PLACE through symlinks (nothing of the reference is
-    copied or edited); only the relative dataset root `../dataset/AnimatedDrawings/preprocessed` (config_stage1.yaml:76)
-    resolves into the temporary tree.  Skipped where the reference checkout is absent (the GPU box of the driver)."""
-    import subprocess
-    import sys
-    from PIL import Image
-    ref = _reference_dir()
-    if ref is None:
-        pytest.skip("reference checkout not present (set DSU_REFERENCE_DIR)")
-    work = tmp_path / "3_style_translator"
-    work.mkdir()
-    for name in ("test_stage1.py", "test_stage2.py", "training", "configs"):
-        os.symlink(os.path.join(ref, name), work / name)
-    root = tmp_path / "dataset" / "AnimatedDrawings" / "preprocessed"
-    uid, h, w, n = "synthetic0001", 64, 48, 3
-    sd1 = synth.to_torch_state_dict(synth.make_state_dict(1, out_gain=0.25))
-    sd2 = synth.to_torch_state_dict(synth.make_state_dict(2, out_gain=0.25))
-    stacks = synth.write_character_tree(str(root), uid, {"dab": n}, h, w, seed=5, state_dicts=(sd1, sd2))
-    color, pos, edge = stacks["dab"]
-    repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    env = dict(os.environ, PYTHONPATH=repo + os.pathsep + os.environ.get("PYTHONPATH", ""), DSU_PRECISION="fp16x3")
-    for script in ("test_stage1.py", "test_stage2.py"):
-        r = subprocess.run([sys.executable, "-m", "drawingspinup_b200.run", str(work / script), "--uid", uid],
-                           env=env, capture_output=True, text=True, timeout=600)
-        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-4000:]
-        assert "Testing finished" in r.stdout
-    base = root / uid / "mesh" / "blender_render" / "dab"
-    got1 = np.stack([np.array(Image.open(base / "res_stage1_mask_pos" / ("%04d.png" % i))) for i in range(n)])
-    got2 = np.stack([np.array(Image.open(base / "res_stage2_mask_pos_edge" / ("%04d.png" % i))) for i in range(n)])
-    with torch.no_grad():
-        x1 = torch.from_numpy(np.stack([rp.frame_to_tensor(color[i], pos[i])[0] for i in range(n)]))
-        y1 = rp.generator_j_ric_forward(sd1, x1, use_torchvision=True)
-        want1 = np.stack([rp.compose_rgba(y1[i].numpy(), rp.frame_to_tensor(color[i], pos[i])[1]) for i in range(n)])
-        # stage 2 reads stage 1's PNGs back from disk (config_stage2.yaml:61 pre_dir) - use the bytes the engine wrote
-        x2 = torch.from_numpy(np.stack([rp.frame_to_tensor(got1[i], pos[i], edge[i])[0] for i in range(n)]))
-        y2 = rp.generator_j_forward(sd2, x2)
-        want2 = np.stack([rp.compose_rgba(y2[i].numpy(), rp.frame_to_tensor(got1[i], pos[i])[1]) for i in range(n)])
-    for got, want in ((got1, want1), (got2, want2)):
-        d = np.abs(got.astype(np.int32) - want.astype(np.int32))
-        assert got.shape == want.shape and d.max() <= 1 and (d > 0).mean() < 0.01
+# ------------------------------------------------------------------ the reference scripts' frame loop on the engine
+def test_engine_reproduces_reference_script_frames(dev, golden_dir, monkeypatch):
+    """SURVEY.md section 4 item 4: the frames the unmodified test_stage1.py / test_stage2.py wrote for a synthetic 3-frame
+    character on the reference's own models (recorded by oracle/make_golden.py) are what the engine gives in their place
+    (<= 1 LSB).  The engine classes come from a ``training.models`` module rebound by install() and are built as
+    build_model builds them (trainers.py:33-35); every frame then goes through the scripts' loop: dataset transform,
+    forward, to_image_space, mask as alpha.  Stage 2 reads the stage-1 frames the reference wrote (config_stage2.yaml:61
+    pre_dir), so both stages are compared on identical inputs."""
+    import types
+    g = np.load(os.path.join(golden_dir, "reference_scripts.npz"))
+    color, pos, edge = g["color"], g["pos"], g["edge"]
+    monkeypatch.setenv("DSU_PRECISION", "fp16x3")
+    models = dsu.install(types.ModuleType("training.models"))
+    for stage, name, pre, want in ((1, "GeneratorJ_RIC", color, g["stage1"]), (2, "GeneratorJ", g["stage1"], g["stage2"])):
+        gen = getattr(models, name)(**DEFAULT_ARGS).to(dev)
+        gen.load_state_dict(synth.to_torch_state_dict(synth.make_state_dict(stage, out_gain=float(g["out_gain"]))))
+        gen.eval()
+        got = []
+        with torch.no_grad():
+            for i in range(color.shape[0]):
+                x, mask = rp.frame_to_tensor(pre[i], pos[i], edge[i] if stage == 2 else None)
+                y = gen(torch.from_numpy(x)[None].to(dev))[0]
+                got.append(rp.compose_rgba(y.cpu().numpy(), mask))
+        d = np.abs(np.stack(got).astype(np.int32) - want.astype(np.int32))
+        assert d.max() <= 1 and (d > 0).mean() < 0.01, (stage, d.max(), (d > 0).mean())

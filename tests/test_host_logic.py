@@ -106,40 +106,33 @@ def test_install_rebinds_reference_names():
     assert isinstance(model, dsu.GeneratorJ_RIC)
 
 
-def test_real_build_model_returns_engine_classes():
-    """The real factory seam (trainers.py:33-35) with the real reference modules: after install() the UNMODIFIED
-    ``training.trainers.build_model`` constructs the engine classes, and a state dict produced by the reference's own
-    classes loads strictly (same 89 keys, same order); uninstall() restores the reference classes.  Needs the reference
-    checkout (present in the build container; skipped elsewhere)."""
-    ref = os.environ.get("DSU_REFERENCE_DIR", "/root/reference/3_style_translator")
-    if not os.path.exists(os.path.join(ref, "training", "trainers.py")):
-        pytest.skip("reference checkout not present")
-    saved = {k: v for k, v in sys.modules.items() if k == "training" or k.startswith("training.")}
-    for k in saved:
-        del sys.modules[k]
-    sys.path.insert(0, ref)
-    try:
-        import importlib
-        m = importlib.import_module("training.models")
-        t = importlib.import_module("training.trainers")
-        args = dict(DEFAULT_ARGS)
-        ref_models = {name: t.build_model(name, dict(args), "cpu") for name in ("GeneratorJ", "GeneratorJ_RIC")}
-        assert all(type(v).__module__ == "training.models" for v in ref_models.values())
-        dsu.install(m)
-        for name, cls in (("GeneratorJ", dsu.GeneratorJ), ("GeneratorJ_RIC", dsu.GeneratorJ_RIC)):
-            eng = t.build_model(name, dict(args), "cpu")            # the unmodified factory, call-time getattr
-            assert type(eng) is cls
-            sd = ref_models[name].state_dict()
-            eng.load_state_dict(sd)                                   # strict
-            assert list(eng.state_dict().keys()) == list(sd.keys())
-            assert all(torch.equal(a, b) for a, b in zip(eng.state_dict().values(), sd.values()))
-        dsu.uninstall(m)
-        assert type(t.build_model("GeneratorJ", dict(args), "cpu")).__module__ == "training.models"
-    finally:
-        sys.path.remove(ref)
-        for k in [k for k in sys.modules if k == "training" or k.startswith("training.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+def test_factory_seam_builds_engine_classes_with_reference_state_dict_layout(golden_dir):
+    """The factory seam (trainers.py:33-35, ``getattr(training.models, name)(**args).to(device)``): after install() it
+    constructs the engine classes, whose state dicts have exactly the layout of the models the reference's own
+    build_model makes (89 keys in the same order, same shapes and dtypes; recorded by oracle/make_golden.py) and load
+    such a state dict strictly; uninstall() restores the module's own classes."""
+    import json
+    from collections import OrderedDict
+    with open(os.path.join(golden_dir, "reference_state_dict_layout.json")) as f:
+        g = json.load(f)
+    assert g["args"] == DEFAULT_ARGS
+    originals = {name: type(name, (), {}) for name in ("GeneratorJ", "GeneratorJ_RIC")}
+    m = types.ModuleType("training.models")
+    m.__dict__.update(originals)
+    dsu.install(m)
+    gen = torch.Generator().manual_seed(0)
+    for name, cls in (("GeneratorJ", dsu.GeneratorJ), ("GeneratorJ_RIC", dsu.GeneratorJ_RIC)):
+        eng = getattr(m, name)(**dict(g["args"])).to("cpu")
+        assert type(eng) is cls
+        layout = g["models"][name]
+        assert len(layout) == 89
+        assert [[k, list(v.shape), str(v.dtype)] for k, v in eng.state_dict().items()] == layout
+        sd = OrderedDict((k, torch.randint(0, 100, s, generator=gen) if dt == "torch.int64" else torch.randn(s, generator=gen))
+                         for k, s, dt in layout)
+        eng.load_state_dict(sd)                                       # strict
+        assert all(torch.equal(a, b) for a, b in zip(eng.state_dict().values(), sd.values()))
+    dsu.uninstall(m)
+    assert all(getattr(m, name) is cls for name, cls in originals.items())
 
 
 def test_launcher_runs_script_with_rebound_classes(tmp_path, monkeypatch, capsys):
